@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the fused CollectiveCrossing step kernel (contract: see the task statement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[1] geometry and policy — the README 12x8 grid
@@ -28,6 +28,7 @@ for p in (str(ROOT), str(ROOT / "tests")):
 
 METRIC = "agent_steps_per_sec"
 UNIT = "agent-steps/s"
+DUMP_BYTES = 48 * 10**6   # --dump-outputs: at most this many bytes of .npy data
 
 
 def parse():
@@ -45,7 +46,15 @@ def parse():
     ap.add_argument("--e2e-steps", type=int, default=24)
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary measurements")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (obs, reward, agent_flags, env_flags, actions) as DIR/<name>.npy "
+                         "in float32; above %d MB a fixed, seeded sample of envs (rank 0's shard with --gpus > 1)" % (DUMP_BYTES // 10**6))
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def workload_config():
@@ -345,6 +354,25 @@ def desynchronise(env, torch):
         env.step_count.copy_(torch.randint(0, hi, (env.num_envs,), generator=g, device=env.device, dtype=torch.int32))
 
 
+def dump_outputs(out_dir, outputs, torch):
+    """Write the step outputs in `outputs` (name -> device tensor with the env index first, or None) as out_dir/<name>.npy in
+    float32.  Where they exceed DUMP_BYTES, the same envs of every output are kept: a sorted sample drawn with a fixed seed, so
+    that two builds run with the same arguments can be compared file for file."""
+    import numpy as np
+
+    outputs = {k: v for k, v in outputs.items() if v is not None}
+    n = next(iter(outputs.values())).shape[0]
+    per_env = sum(4 * v[0].numel() for v in outputs.values())
+    keep = min(n, DUMP_BYTES // per_env)
+    idx = None
+    if keep < n:
+        idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, keep, replace=False))).to(next(iter(outputs.values())).device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in outputs.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), (v if idx is None else v.index_select(0, idx)).float().cpu().numpy())
+    print(f"dumped the last timed step's outputs of {keep} of {n} envs to {out_dir}", file=sys.stderr)
+
+
 def median(vals):
     v = sorted(vals)
     return v[len(v) // 2] if len(v) % 2 else 0.5 * (v[len(v) // 2 - 1] + v[len(v) // 2])
@@ -465,8 +493,9 @@ def run_ours(args):
     sampler = ClockSampler(local) if rank == 0 else None
     for _ in range(args.warmup):
         env.step(policy=args.policy)
-    if T > 1:
-        env.rollout_trajectory(T, policy=args.policy)   # allocates the [T, N, ...] output buffers, warms the fused launch
+    traj = None
+    if T > 1:   # allocates the [T, N, ...] output buffers, which every timed launch of T steps refills; warms the fused launch
+        traj = env.rollout_trajectory(T, policy=args.policy)
     if world > 1:
         sharded.global_stats_device()                   # warms the NCCL communicator
     torch.cuda.synchronize()
@@ -488,6 +517,11 @@ def run_ours(args):
     ms = median(rep_ms)
     env.check_error()
     kernel_name = env.last_kernel_name
+    if args.dump_outputs and rank == 0:
+        last = {"obs": env.obs, "reward": env.reward, "agent_flags": env.agent_flags, "env_flags": env.env_flags, "actions": env.actions_out}
+        if T > 1 and args.steps % T == 0:   # the last timed step was the last step of a fused launch
+            last = {k: None if traj[k] is None else traj[k][-1] for k in last}
+        dump_outputs(args.dump_outputs, last, torch)
 
     # episode statistics of the job: at world > 1 the tensor the in-loop all-reduce left on the device
     st = sharded.stats_from_tensor(stats_t) if stats_t is not None else sharded.global_stats()

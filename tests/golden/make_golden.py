@@ -6,7 +6,8 @@ Each file holds, for a handful of envs, the state after ``reset(seed)``, the act
 everything ``CollectiveCrossingEnv.step`` returned at every step, in the batched encoding of
 ``include/ccb200.h`` (see ``oracle/refrun.py:record``).  ``cassette_basic.npz`` /
 ``cassette_regression.npz`` are the reference's own golden cassettes
-(tests/fixtures/trajectories/golden/*.json) converted to the same encoding.
+(tests/fixtures/trajectories/golden/*.json) converted to the same encoding; the two JSON files are stored
+next to them as they are.
 The reference cannot travel to the GPU box, these files do.
 """
 
@@ -88,6 +89,7 @@ def main() -> None:
     for src, dst in (("golden_basic_trajectory.json", "cassette_basic"), ("regression_test.json", "cassette_regression")):
         rec = convert_cassette(gold / src)
         np.savez_compressed(OUT / f"{dst}.npz", seeds=np.array([42], np.int64), **rec)
+        (OUT / src).write_bytes((gold / src).read_bytes())   # the cassette itself, for tests/test_cassette_cpu.py
         print(f"{dst}: {rec['actions'].shape}")
 
 

@@ -5,6 +5,8 @@ import subprocess
 import sys
 from pathlib import Path
 
+import pytest
+
 ROOT = Path(__file__).resolve().parents[1]
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
@@ -32,6 +34,43 @@ def test_other_ranks_of_the_reference_arm_exit_silently():
     out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],
                          capture_output=True, text=True, timeout=60, cwd=ROOT, env={**__import__("os").environ, "RANK": "1", "WORLD_SIZE": "2"})
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+@pytest.mark.parametrize("args", [["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_refuses_arguments_it_cannot_honour(args):
+    out = subprocess.run([sys.executable, str(ROOT / "bench.py"), *args], capture_output=True, text=True, timeout=60, cwd=ROOT)
+    assert out.returncode == 2 and out.stdout == "" and "error:" in out.stderr
+
+
+DUMP_TWICE = """
+import sys
+from pathlib import Path
+import torch
+import bench
+n, out = 200_000, Path(sys.argv[1])
+env = torch.arange(n, dtype=torch.float32)
+outputs = {"obs": env[:, None, None].expand(n, 8, 38).contiguous(), "reward": env[:, None].expand(n, 8).contiguous(),
+           "env_flags": env.clone(), "agent_info": None}
+for run in ("a", "b"):
+    bench.dump_outputs(out / run, outputs, torch)
+"""
+
+
+def test_dump_sample_keeps_the_same_envs_in_every_output(tmp_path):
+    """Outputs above the size limit are cut to one seeded sample of envs, the same for every array and every run.  (In a
+    subprocess: torch's worker threads would otherwise be running when later tests fork.)"""
+    import numpy as np
+
+    out = subprocess.run([sys.executable, "-c", DUMP_TWICE, str(tmp_path)], capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    got = {run: {k: np.load(tmp_path / run / f"{k}.npy") for k in ("obs", "reward", "env_flags")} for run in ("a", "b")}
+    assert not (tmp_path / "a" / "agent_info.npy").exists()
+    ids = got["a"]["env_flags"]
+    assert sum(v.nbytes for v in got["a"].values()) <= 48 * 10**6 and 0 < len(ids) < 200_000
+    assert np.all(np.diff(ids) > 0) and ids[-1] > len(ids)       # sorted, distinct, not a prefix
+    assert (got["a"]["obs"] == ids[:, None, None]).all() and (got["a"]["reward"] == ids[:, None]).all()
+    for k in got["a"]:
+        assert np.array_equal(got["a"][k], got["b"][k]), k
 
 
 def test_committed_bench_record_carries_the_contract():
