@@ -105,6 +105,8 @@ EXPORTS = {
     "cc_last_host_call": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "cc_timing_begin": (C.c_int, [_P, _P]),
     "cc_timing_end": (C.c_int, [_P, _P, C.POINTER(C.c_float)]),
+    "cc_device_alloc": (C.c_int, [C.c_int, C.c_size_t, C.POINTER(_P), C.POINTER(_I32)]),
+    "cc_device_free": (C.c_int, [_P]),
     "cc_last_error": (C.c_char_p, []),
     "cc_abi_version": (C.c_int, []),
 }

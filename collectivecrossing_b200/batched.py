@@ -12,6 +12,14 @@ Encoding (see the ``CC_*`` enums in the header, mirrored in ``_abi``):
   ``step_count`` int32 [N]; ``episode_return`` float32 [N]
 * agent order is the reference's: ``boarding_0..B-1`` then ``exiting_0..E-1``
 * outputs are overwritten in place by every step (the returned ``StepOutput`` aliases them)
+
+The output tensors (``obs``, ``reward``, flags, infos, applied actions, and the ``[T, N, ...]`` buffers of
+``rollout_trajectory``) live in memory from the library's ``cc_device_alloc``: compressible device memory where the
+GPU grants it (``outputs_compressed``), else plain device memory.  Compression changes no value; it cuts the DRAM
+bytes of the very regular observation rows.  Two limits follow: ``torch.cuda.memory_allocated`` does not count these
+tensors, and they cannot be shared through CUDA IPC (``torch.multiprocessing``).  Releasing one waits for the
+device, like ``cudaFree``, so do not drop the last reference to an env or its output tensors while capturing a CUDA
+graph.  The state tensors are ordinary torch allocations.
 """
 
 from __future__ import annotations
@@ -28,6 +36,27 @@ from .lowering import lower_config
 _OBS_TORCH = {"none": (None, _abi.OBS_NONE), "int8": (torch.int8, _abi.OBS_INT8), "float32": (torch.float32, _abi.OBS_FP32),
               "table": (torch.int8, _abi.OBS_TABLE)}
 _REW_TORCH = {"float32": (torch.float32, _abi.REWARD_F32), "float64": (torch.float64, _abi.REWARD_F64)}
+_TYPESTR = {torch.float32: "<f4", torch.float64: "<f8", torch.int8: "|i1", torch.uint8: "|u1"}
+
+
+class _DeviceBuffer:
+    """Zeroed memory from ``cc_device_alloc`` exposed through ``__cuda_array_interface__``.  A tensor made from it
+    holds a reference to it, so the memory goes back to the library (``cc_device_free``) when the last view dies."""
+
+    def __init__(self, lib, device_index: int, shape: tuple, dtype: torch.dtype):
+        nbytes = dtype.itemsize
+        for d in shape:
+            nbytes *= d
+        self._lib, self.ptr = lib, None
+        ptr, compressed = C.c_void_p(), C.c_int32()
+        _native.check(lib.cc_device_alloc(device_index, max(nbytes, 1), C.byref(ptr), C.byref(compressed)))
+        self.ptr, self.compressed = ptr.value, bool(compressed.value)
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": _TYPESTR[dtype], "data": (ptr.value, False),
+                                         "strides": None, "version": 2}
+
+    def __del__(self):
+        if self.ptr is not None:
+            self._lib.cc_device_free(self.ptr)
 
 
 @dataclass
@@ -121,12 +150,13 @@ class BatchedCollectiveCrossing:
         self.episode_return = torch.zeros((n,), dtype=torch.float32, device=dev)
         # last axis of the obs output: the reference's row (6+4A) or one block of the compact table
         self.obs_width = 4 if self.obs_code == _abi.OBS_TABLE else self.obs_len
-        self.obs = None if self.obs_code == _abi.OBS_NONE else torch.zeros((n, a, self.obs_width), dtype=self.obs_torch_dtype, device=dev)
-        self.reward = torch.zeros((n, a), dtype=self.reward_torch_dtype, device=dev)
-        self.agent_flags = torch.zeros((n, a), dtype=torch.uint8, device=dev)
-        self.agent_info = torch.zeros((n, a), dtype=torch.uint8, device=dev) if with_info else None
-        self.env_flags = torch.zeros((n,), dtype=torch.uint8, device=dev)
-        self.actions_out = torch.zeros((n, a), dtype=torch.int8, device=dev)
+        self.outputs_compressed = True   # cleared by _output_tensor when the device does not grant compressible memory
+        self.obs = None if self.obs_code == _abi.OBS_NONE else self._output_tensor((n, a, self.obs_width), self.obs_torch_dtype)
+        self.reward = self._output_tensor((n, a), self.reward_torch_dtype)
+        self.agent_flags = self._output_tensor((n, a), torch.uint8)
+        self.agent_info = self._output_tensor((n, a), torch.uint8) if with_info else None
+        self.env_flags = self._output_tensor((n,), torch.uint8)
+        self.actions_out = self._output_tensor((n, a), torch.int8)
 
         handle = C.c_void_p()
         _native.check(self._lib.cc_create(C.byref(self.cfg), n, self.device_index, self.global_env_offset, self.seed, C.byref(handle)))
@@ -153,6 +183,14 @@ class BatchedCollectiveCrossing:
     def last_kernel_name(self) -> str:
         """Instantiation the last ``step`` launch ran, e.g. ``ccb::cc_step_tpe_kernel<8,4>``."""
         return self._lib.cc_last_kernel_name(self._h).decode()
+
+    def _output_tensor(self, shape: tuple, dtype: torch.dtype) -> torch.Tensor:
+        """A zeroed output tensor in memory from ``cc_device_alloc`` (compressible where the device grants it)."""
+        buf = _DeviceBuffer(self._lib, self.device_index, shape, dtype)
+        self.outputs_compressed = self.outputs_compressed and buf.compressed
+        t = torch.as_tensor(buf)
+        assert t.device == self.x.device and t.dtype == dtype and t.is_contiguous()
+        return t
 
     # ------------------------------------------------------------------------------------------
     def close(self) -> None:
@@ -284,14 +322,14 @@ class BatchedCollectiveCrossing:
             raise ValueError("n_steps must be positive")
         buf = getattr(self, "_traj", None)
         if buf is None or buf["reward"].shape[0] != T:
-            dev = self.device
+            out = self._output_tensor
             buf = self._traj = dict(
-                obs=None if self.obs is None else torch.zeros((T, n, a, self.obs_width), dtype=self.obs_torch_dtype, device=dev),
-                reward=torch.zeros((T, n, a), dtype=self.reward_torch_dtype, device=dev),
-                agent_flags=torch.zeros((T, n, a), dtype=torch.uint8, device=dev),
-                agent_info=None if self.agent_info is None else torch.zeros((T, n, a), dtype=torch.uint8, device=dev),
-                env_flags=torch.zeros((T, n), dtype=torch.uint8, device=dev),
-                actions=torch.zeros((T, n, a), dtype=torch.int8, device=dev))
+                obs=None if self.obs is None else out((T, n, a, self.obs_width), self.obs_torch_dtype),
+                reward=out((T, n, a), self.reward_torch_dtype),
+                agent_flags=out((T, n, a), torch.uint8),
+                agent_info=None if self.agent_info is None else out((T, n, a), torch.uint8),
+                env_flags=out((T, n), torch.uint8),
+                actions=out((T, n, a), torch.int8))
         io = _abi.CCStepIO()
         code = _policy_code(policy)
         if code == _abi.POLICIES["external"]:

@@ -13,6 +13,8 @@
 #include <utility>
 #include <vector>
 
+#include <cuda.h>   // driver types of cc_device_alloc (the functions are resolved at run time)
+
 #include "cc_internal.h"
 #include "cc_workers.h"
 #include "cc_kernel_tpe.cuh"   // KParams, layout constants (no kernel is instantiated in this file)
@@ -40,6 +42,48 @@ size_t obs_env_bytes(int A, int obs_dtype) {
     if (obs_dtype == CC_OBS_TABLE) return 4 * (size_t)A;
     return is_rows(obs_dtype) ? (size_t)A * (6 + 4 * (size_t)A) * (size_t)obs_dtype : 0;
 }
+
+// Driver entry points of cc_device_alloc, resolved through the runtime: the library links the static runtime, not libcuda.
+struct DriverApi {
+    bool ok = false;
+    decltype(&::cuDeviceGetAttribute) cuDeviceGetAttribute = nullptr;
+    decltype(&::cuMemGetAllocationGranularity) cuMemGetAllocationGranularity = nullptr;
+    decltype(&::cuMemCreate) cuMemCreate = nullptr;
+    decltype(&::cuMemGetAllocationPropertiesFromHandle) cuMemGetAllocationPropertiesFromHandle = nullptr;
+    decltype(&::cuMemAddressReserve) cuMemAddressReserve = nullptr;
+    decltype(&::cuMemMap) cuMemMap = nullptr;
+    decltype(&::cuMemSetAccess) cuMemSetAccess = nullptr;
+    decltype(&::cuMemUnmap) cuMemUnmap = nullptr;
+    decltype(&::cuMemAddressFree) cuMemAddressFree = nullptr;
+    decltype(&::cuMemRelease) cuMemRelease = nullptr;
+};
+
+template <typename F>
+bool driver_entry(const char *name, F &fn) {
+    cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+    void *p = nullptr;
+    if (cudaGetDriverEntryPointByVersion(name, &p, 12000, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) return false;
+    fn = reinterpret_cast<F>(p);
+    return true;
+}
+
+const DriverApi &driver_api() {
+    static const DriverApi api = [] {
+        DriverApi d;
+        d.ok = driver_entry("cuDeviceGetAttribute", d.cuDeviceGetAttribute) && driver_entry("cuMemGetAllocationGranularity", d.cuMemGetAllocationGranularity) &&
+               driver_entry("cuMemCreate", d.cuMemCreate) && driver_entry("cuMemGetAllocationPropertiesFromHandle", d.cuMemGetAllocationPropertiesFromHandle) &&
+               driver_entry("cuMemAddressReserve", d.cuMemAddressReserve) && driver_entry("cuMemMap", d.cuMemMap) &&
+               driver_entry("cuMemSetAccess", d.cuMemSetAccess) && driver_entry("cuMemUnmap", d.cuMemUnmap) &&
+               driver_entry("cuMemAddressFree", d.cuMemAddressFree) && driver_entry("cuMemRelease", d.cuMemRelease);
+        return d;
+    }();
+    return api;
+}
+
+// live allocations of cc_device_alloc; mapped = 0: plain cudaMalloc memory
+struct DeviceAlloc { void *ptr; size_t mapped; unsigned long long handle; int device; };
+std::mutex g_alloc_mu;
+std::vector<DeviceAlloc> g_allocs;
 
 }  // namespace
 
@@ -864,6 +908,109 @@ int cc_timing_end(cc_handle *h, void *stream, float *total_ms) {
     CC_CUDA(cudaEventRecord(h->ev1, static_cast<cudaStream_t>(stream)));
     CC_CUDA(cudaEventSynchronize(h->ev1));
     CC_CUDA(cudaEventElapsedTime(total_ms, h->ev0, h->ev1));
+    return CC_OK;
+}
+
+int cc_device_alloc(int device, size_t bytes, void **ptr, int32_t *compressed) {
+    if (!ptr || !compressed) return cc_fail(CC_ERR_INVALID_ARG, "cc_device_alloc: null pointer");
+    if (bytes == 0) return cc_fail(CC_ERR_INVALID_ARG, "cc_device_alloc: bytes must be positive");
+    *ptr = nullptr;
+    *compressed = 0;
+    int count = 0;
+    CC_CUDA(cudaGetDeviceCount(&count));
+    if (device < 0 || device >= count) return cc_fail(CC_ERR_INVALID_ARG, "device %d out of range (%d visible)", device, count);
+    DeviceGuard guard(device);
+    const DriverApi &d = driver_api();
+    void *p = nullptr;
+    size_t mapped = 0;
+    unsigned long long handle = 0;
+    int supported = 0;
+    if (d.ok && d.cuDeviceGetAttribute(&supported, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, device) == CUDA_SUCCESS && supported) {
+        CUmemAllocationProp prop = {};
+        prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+        prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+        prop.location.id = device;
+        prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+        size_t gran = 0;
+        CUmemGenericAllocationHandle h = 0;
+        CUmemAllocationProp got = {};
+        if (d.cuMemGetAllocationGranularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED) == CUDA_SUCCESS && gran) {
+            const size_t size = (bytes + gran - 1) / gran * gran;
+            // the driver may grant plain memory (or none) instead: then this buffer comes from cudaMalloc
+            if (d.cuMemCreate(&h, size, &prop, 0) == CUDA_SUCCESS) {
+                CUdeviceptr va = 0;
+                CUmemAccessDesc acc = {};
+                acc.location = prop.location;
+                acc.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+                if (d.cuMemGetAllocationPropertiesFromHandle(&got, h) == CUDA_SUCCESS && got.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC &&
+                    d.cuMemAddressReserve(&va, size, gran, 0, 0) == CUDA_SUCCESS) {
+                    if (d.cuMemMap(va, size, 0, h, 0) == CUDA_SUCCESS) {
+                        if (d.cuMemSetAccess(va, size, &acc, 1) == CUDA_SUCCESS) {
+                            p = reinterpret_cast<void *>(va);
+                            mapped = size;
+                            handle = h;
+                        } else {
+                            d.cuMemUnmap(va, size);
+                        }
+                    }
+                    if (!p) d.cuMemAddressFree(va, size);
+                }
+                if (!p) d.cuMemRelease(h);
+            }
+        }
+    }
+    if (!p) {
+        const cudaError_t e = cudaMalloc(&p, bytes);
+        if (e != cudaSuccess) return cc_fail(CC_ERR_NOMEM, "cudaMalloc(%zu): %s", bytes, cudaGetErrorString(e));
+    }
+    // Zero-initialised, like the tensors this memory replaces.  The fill goes to the legacy default stream, which a
+    // non-blocking caller stream (torch.cuda.Stream()) does not wait for: it must be complete before this returns, or a
+    // kernel launched right after on such a stream could race with it and have its outputs zeroed.
+    cudaError_t e = cudaMemsetAsync(p, 0, bytes, cudaStreamLegacy);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(cudaStreamLegacy);
+    if (e == cudaSuccess) {
+        std::lock_guard<std::mutex> lock(g_alloc_mu);
+        g_allocs.push_back({p, mapped, handle, device});
+    } else {
+        if (mapped) {
+            d.cuMemUnmap(reinterpret_cast<CUdeviceptr>(p), mapped);
+            d.cuMemAddressFree(reinterpret_cast<CUdeviceptr>(p), mapped);
+            d.cuMemRelease(handle);
+        } else {
+            cudaFree(p);
+        }
+        return cc_fail(CC_ERR_CUDA, "zero fill of %zu bytes: %s", bytes, cudaGetErrorString(e));
+    }
+    *ptr = p;
+    *compressed = mapped ? 1 : 0;
+    return CC_OK;
+}
+
+int cc_device_free(void *ptr) {
+    if (!ptr) return CC_OK;
+    DeviceAlloc a = {};
+    {
+        std::lock_guard<std::mutex> lock(g_alloc_mu);
+        auto it = std::find_if(g_allocs.begin(), g_allocs.end(), [&](const DeviceAlloc &x) { return x.ptr == ptr; });
+        if (it == g_allocs.end()) return cc_fail(CC_ERR_INVALID_ARG, "cc_device_free: %p was not allocated by cc_device_alloc", ptr);
+        a = *it;
+    }
+    DeviceGuard guard(a.device);
+    if (!a.mapped) {
+        CC_CUDA(cudaFree(ptr));
+    } else {
+        // cudaFree waits for the device before it releases memory; unmapping must too (a launch queued on any stream
+        // may still write here).  The library does not know which streams used the buffer, so it waits for all of them.
+        CC_CUDA(cudaDeviceSynchronize());
+        const DriverApi &d = driver_api();
+        const CUdeviceptr va = reinterpret_cast<CUdeviceptr>(ptr);
+        if (d.cuMemUnmap(va, a.mapped) != CUDA_SUCCESS || d.cuMemAddressFree(va, a.mapped) != CUDA_SUCCESS || d.cuMemRelease(a.handle) != CUDA_SUCCESS)
+            return cc_fail(CC_ERR_CUDA, "cc_device_free: releasing the compressible allocation at %p failed", ptr);
+    }
+    // forgotten only once released: a failed free (e.g. during stream capture) can be repeated
+    std::lock_guard<std::mutex> lock(g_alloc_mu);
+    auto it = std::find_if(g_allocs.begin(), g_allocs.end(), [&](const DeviceAlloc &x) { return x.ptr == ptr; });
+    if (it != g_allocs.end()) g_allocs.erase(it);
     return CC_OK;
 }
 

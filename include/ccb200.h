@@ -29,6 +29,7 @@
 #ifndef CCB200_H
 #define CCB200_H
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -324,6 +325,18 @@ int cc_last_host_call(const cc_handle *h, int64_t out[5]);
  * measured with CUDA events on the launching stream */
 int cc_timing_begin(cc_handle *h, void *stream);
 int cc_timing_end(cc_handle *h, void *stream, float *total_ms);
+
+/* --- output buffers -------------------------------------------------------------------- */
+/* `bytes` of zeroed device memory on `device` for step outputs (the zero fill is complete when the call returns).  Where the device supports compressible memory
+ * (CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED) and grants it, the memory is compressible (cuMemCreate with
+ * CU_MEM_ALLOCATION_COMP_GENERIC): the hardware compresses it between L2 and DRAM, which cuts the DRAM bytes of the
+ * very regular float32 observation rows; every value read or written is unchanged.  Otherwise it is cudaMalloc memory.
+ * *compressed is 1 for compressible memory, else 0.  Not shareable through CUDA IPC.  Free with cc_device_free. */
+int cc_device_alloc(int device, size_t bytes, void **ptr, int32_t *compressed);
+/* Waits for the whole device (like cudaFree), then releases memory from cc_device_alloc (NULL: no-op).  It therefore
+ * fails while a stream of the device is being captured into a CUDA graph; the memory then stays allocated and the call
+ * can be repeated after the capture. */
+int cc_device_free(void *ptr);
 
 const char *cc_last_error(void);
 int cc_abi_version(void);
