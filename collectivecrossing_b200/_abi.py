@@ -22,6 +22,7 @@ O_ACTIVE, O_TERMINATED, O_TRUNCATED, O_ALIVE_PREV, O_TERM_VALUE, O_TRUNC_VALUE, 
 I_IN_TRAM_AREA, I_AT_DOOR, I_ACTIVE, I_AT_DESTINATION = 1, 2, 4, 8
 E_TERMINATED_ALL, E_TRUNCATED_ALL, E_WAS_RESET = 1, 2, 4
 KERNEL_VARIANTS = {"auto": 0, "lanes": 1, "threads": 2}
+RESET_RNG = {"philox": 0, "numpy": 1}
 
 
 class CCConfig(C.Structure):
@@ -83,6 +84,8 @@ EXPORTS = {
     "cc_get_rng_state": (C.c_int, [_P, _P, _P]),
     "cc_set_rng_state": (C.c_int, [_P, _P, _P]),
     "cc_rng_seeded": (_I32, [_P]),
+    "cc_set_reset_rng": (C.c_int, [_P, _I32]),
+    "cc_reset_rng": (_I32, [_P]),
     "cc_rollout": (C.c_int, [_P, C.POINTER(CCStepIO), _I32, _P]),
     "cc_rollout_fused": (C.c_int, [_P, C.POINTER(CCStepIO), _I32, _P]),
     "cc_reset": (C.c_int, [_P, _P, _P, _I32, _P]),

@@ -114,11 +114,17 @@ class BatchedCollectiveCrossing:
     Parameters mirror ``CollectiveCrossingEnv(config)``; ``global_env_offset`` is this shard's
     first env in the whole job (the counter-based RNG is keyed on the global env index, so a run
     sharded over 8 GPUs reproduces the 1-GPU run env by env).
+
+    ``reset_rng`` chooses where unseeded placements (the auto-reset and ``reset(mask)``) come from: "philox"
+    (default, counter-based) or "numpy": the reference's ``reset()`` without a seed, env n continuing the numpy
+    generator ``reset_seeded`` gave it — N envs seeded once and stepped with auto-reset then reproduce N reference
+    envs episode after episode.  In "numpy" mode a call that may place envs raises until ``reset_seeded(seeds)`` or
+    ``load_state`` has seeded the generators.
     """
 
     def __init__(self, config: Any, num_envs: int, device: Any = "cuda:0", *, seed: int = 0,
                  global_env_offset: int = 0, obs_dtype: str = "float32", reward_dtype: str = "float32",
-                 auto_reset: bool = True, with_info: bool = False, kernel: str = "auto"):
+                 auto_reset: bool = True, with_info: bool = False, kernel: str = "auto", reset_rng: str = "philox"):
         self._lib = _native.library()  # raises ImportError when the CUDA library is not built
         if not torch.cuda.is_available():
             raise RuntimeError("collectivecrossing_b200 needs a CUDA device (no CPU fallback exists)")
@@ -126,6 +132,8 @@ class BatchedCollectiveCrossing:
             raise ValueError(f"obs_dtype must be one of {list(_OBS_TORCH)}")
         if reward_dtype not in _REW_TORCH:
             raise ValueError(f"reward_dtype must be one of {list(_REW_TORCH)}")
+        if reset_rng not in _abi.RESET_RNG:
+            raise ValueError(f"reset_rng must be one of {list(_abi.RESET_RNG)}")
         self.config = config
         self.cfg = config if isinstance(config, _abi.CCConfig) else lower_config(config)
         self.device = torch.device(device)
@@ -165,6 +173,13 @@ class BatchedCollectiveCrossing:
                                                 self.step_count.data_ptr(), self.episode_return.data_ptr()))
         self._io = _abi.CCStepIO()
         self.set_kernel(kernel)
+        _native.check(self._lib.cc_set_reset_rng(self._h, _abi.RESET_RNG[reset_rng]))
+
+    @property
+    def reset_rng(self) -> str:
+        """Where unseeded placements come from: "philox" or "numpy" (``cc_reset_rng``)."""
+        code = int(self._lib.cc_reset_rng(self._h))
+        return next(k for k, v in _abi.RESET_RNG.items() if v == code)
 
     def set_kernel(self, kernel: str) -> None:
         """Work mapping of ``step``: "auto" (default), "lanes" (one lane per agent) or "threads" (one

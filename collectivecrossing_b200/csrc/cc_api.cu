@@ -209,6 +209,13 @@ bool tpe_eligible(const cc_handle *h, const cc_step_io *io, long long first) {
     return aligned_to(io->reward, A % 4 == 0 ? 16 : 4) && aligned_to(h->step, 4) && aligned_to(h->ep_ret, 4);
 }
 
+// a call that may place envs in CC_RESET_RNG_NUMPY mode needs seeded generators (like cc_reset_seeded(NULL))
+int check_reset_rng(const cc_handle *h, bool places) {
+    if (places && h->reset_rng == CC_RESET_RNG_NUMPY && !h->gen_seeded)
+        return cc_fail(CC_ERR_INVALID_ARG, "CC_RESET_RNG_NUMPY places envs from the generators cc_reset_seeded(seeds) or cc_set_rng_state seed: seed them first");
+    return CC_OK;
+}
+
 int check_io(const cc_handle *h, const cc_step_io *io) {
     if (!h || !io) return cc_fail(CC_ERR_INVALID_ARG, "null handle or io");
     if (io->policy < CC_POLICY_EXTERNAL || io->policy > CC_POLICY_WAITING) return cc_fail(CC_ERR_INVALID_ARG, "unknown policy %d", io->policy);
@@ -218,7 +225,7 @@ int check_io(const cc_handle *h, const cc_step_io *io) {
     if (io->obs_dtype != CC_OBS_NONE && !io->obs) return cc_fail(CC_ERR_INVALID_ARG, "obs_dtype set but io->obs is null");
     if (io->reward_dtype != CC_REWARD_F32 && io->reward_dtype != CC_REWARD_F64) return cc_fail(CC_ERR_INVALID_ARG, "unknown reward_dtype %d", io->reward_dtype);
     if (!io->reward || !io->agent_flags || !io->env_flags) return cc_fail(CC_ERR_INVALID_ARG, "reward, agent_flags and env_flags are required");
-    return CC_OK;
+    return check_reset_rng(h, io->auto_reset != 0);
 }
 int check_obs_alignment(const cc_step_io *io) {
     if (io->obs && (reinterpret_cast<uintptr_t>(io->obs) & 15)) return cc_fail(CC_ERR_INVALID_ARG, "io->obs must be 16-byte aligned");
@@ -253,6 +260,7 @@ int step_on(cc_handle *h, const cc_step_io *io, cudaStream_t s, const StepArgs &
     p.actions = io->actions; p.order = io->order; p.actions_out = io->actions_out;
     p.obs = io->obs; p.reward = io->reward; p.agent_flags = io->agent_flags; p.agent_info = io->agent_info; p.env_flags = io->env_flags;
     p.policy = io->policy; p.auto_reset = io->auto_reset != 0; p.reward_f64 = io->reward_dtype == CC_REWARD_F64;
+    if (h->reset_rng == CC_RESET_RNG_NUMPY && p.auto_reset) p.gen = h->gen + a.first;   // (env n of the launch: generator first + n)
     const bool can_tpe = a.obs_env_offset == 0 && tpe_eligible(h, io, a.first);
     if (h->variant == CC_KERNEL_THREADS && !can_tpe)
         return cc_fail(CC_ERR_UNSUPPORTED, "CC_KERNEL_THREADS was requested but this step is not eligible (needs at most 8 agents, agent order, "
@@ -581,6 +589,7 @@ int launch_aux(cc_handle *h, int mode, int obs_dtype, bool bitmap, const uint8_t
     KParams p;
     fill_params(h, p, obs_dtype, bitmap, 0, h->n_envs);
     p.mask = mask; p.obs = obs; p.policy = policy; p.actions_out = actions_out;
+    if (mode == ccb::kModeReset && h->reset_rng == CC_RESET_RNG_NUMPY) p.gen = h->gen;
     return cc_launch_lanes(h, p, mode, obs_dtype, s);
 }
 
@@ -776,9 +785,11 @@ int cc_reset(cc_handle *h, const uint8_t *mask, void *obs, int32_t obs_dtype, vo
     if (obs_dtype != CC_OBS_NONE && !obs) return cc_fail(CC_ERR_INVALID_ARG, "obs_dtype set but obs is null");
     if (!obs) obs_dtype = CC_OBS_NONE;
     if (obs && (reinterpret_cast<uintptr_t>(obs) & 15)) return cc_fail(CC_ERR_INVALID_ARG, "obs must be 16-byte aligned");
+    int rc = check_reset_rng(h, true);
+    if (rc != CC_OK) return rc;
     DeviceGuard guard(h->device);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    int rc = launch_aux(h, ccb::kModeReset, obs_dtype, false, mask, obs, CC_POLICY_EXTERNAL, nullptr, s);
+    rc = launch_aux(h, ccb::kModeReset, obs_dtype, false, mask, obs, CC_POLICY_EXTERNAL, nullptr, s);
     if (rc != CC_OK) return rc;
     h->t += 1;
     return mark_order(h, s);
@@ -841,6 +852,13 @@ int cc_set_rng_state(cc_handle *h, const uint64_t *in, void *stream) {
     return mark_order(h, s);
 }
 int32_t cc_rng_seeded(const cc_handle *h) { return (h && h->gen_seeded) ? 1 : 0; }
+int cc_set_reset_rng(cc_handle *h, int32_t source) {
+    if (!h) return cc_fail(CC_ERR_INVALID_ARG, "null handle");
+    if (source != CC_RESET_RNG_PHILOX && source != CC_RESET_RNG_NUMPY) return cc_fail(CC_ERR_INVALID_ARG, "unknown reset generator %d", source);
+    h->reset_rng = source;
+    return CC_OK;
+}
+int32_t cc_reset_rng(const cc_handle *h) { return h ? h->reset_rng : CC_RESET_RNG_PHILOX; }
 
 int cc_stats_read(cc_handle *h, cc_stats *out, void *stream) {
     if (!h || !out) return cc_fail(CC_ERR_INVALID_ARG, "null handle or out");

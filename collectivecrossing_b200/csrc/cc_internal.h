@@ -49,6 +49,7 @@ struct cc_handle {
     int *err = nullptr;
     ccb::Pcg64State *gen = nullptr;  // per-env numpy-compatible generators (allocated on first seeded reset)
     bool gen_seeded = false;
+    int reset_rng = CC_RESET_RNG_PHILOX;   // cc_set_reset_rng: where the unseeded placements come from
     int64_t launches = 0;
     unsigned *tpe_counters = nullptr;   // two work counters of the thread-per-env kernel (launch parity)
     int64_t tpe_launches = 0;

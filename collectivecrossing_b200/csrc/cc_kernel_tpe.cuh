@@ -270,8 +270,11 @@ __device__ __forceinline__ void tpe_emit_blocks_stg(const unsigned *lut, unsigne
     }
 }
 
-template <int A, int OBS>
+// OBSF: the obs dtype, with kNpReset for numpy-mode auto-reset placements
+template <int A, int OBSF>
 __global__ void __launch_bounds__(kTpeThreads, CCB_TPE_MIN_BLOCKS) cc_step_tpe_kernel(const __grid_constant__ KParams p) {
+    constexpr int OBS = OBSF & ~kNpReset;
+    constexpr bool kNp = (OBSF & kNpReset) != 0;
     using L = TpeLayout<A, OBS>;
     using OT = typename L::OT;
     using P2 = typename L::P2;
@@ -651,6 +654,24 @@ __global__ void __launch_bounds__(kTpeThreads, CCB_TPE_MIN_BLOCKS) cc_step_tpe_k
             eflags |= CC_E_WAS_RESET;
             ep_ret = 0.f;
             step = 0;                                               // :97
+          if constexpr (kNp) {
+            // numpy mode: the env's generator (loaded and stored only here), placement of cc_reset_seeded_kernel
+            Pcg64 g = np_load(p.gen[n]);
+#pragma unroll
+            for (int i = 0; i < A; ++i) {
+                int px = 0, py = 0;
+                const bool ok = np_place_agent(g, p, i < p.B, [&](int cx, int cy) {
+                    bool free = true;
+#pragma unroll
+                    for (int j = 0; j < i; ++j) free = free && pos[j] != pack_pos(cx, cy);
+                    return free;
+                }, px, py);
+                if (!ok) errbits |= kErrResetStuck;                 // cap hit: keep the last candidate
+                pos[i] = pack_pos(px, py);
+                fl[i] = CC_F_ACTIVE;
+            }
+            p.gen[n] = np_save(g);
+          } else {
 #pragma unroll
             for (int i = 0; i < A; ++i) {
                 unsigned cand = 0;
@@ -673,6 +694,7 @@ __global__ void __launch_bounds__(kTpeThreads, CCB_TPE_MIN_BLOCKS) cc_step_tpe_k
                 pos[i] = cand;
                 fl[i] = CC_F_ACTIVE;
             }
+          }
         }
 
         if (env_ok) __stcs(reinterpret_cast<unsigned char *>(p.env_flags) + (size_t)tt * (size_t)p.slice_envs + n, (unsigned char)eflags);

@@ -157,8 +157,11 @@ __global__ void __launch_bounds__(256) cc_t2_tables_kernel(const __grid_constant
 
 // BT >= 0: the number of boarding agents is known at compile time (the README crew, 5 + 3: the type of agent k and with it
 // the table half it reads, the boarding / exiting byte masks ... are immediates); BT = -1: any crew (p.B).
-template <int A, int OBS, int BT>
+// OBSF: the obs dtype, with kNpReset for numpy-mode auto-reset placements (instantiated for BT = -1 only)
+template <int A, int OBSF, int BT>
 __global__ void __launch_bounds__(kT2Threads, CCB_T2_MIN_BLOCKS) cc_step_tpe2_kernel(const __grid_constant__ KParams p) {
+    constexpr int OBS = OBSF & ~kNpReset;
+    constexpr bool kNp = (OBSF & kNpReset) != 0;
     using L = T2Layout<A, OBS>;
     const int B = BT >= 0 ? BT : p.B;
     static_assert(A >= 1 && A <= 8, "thread-per-env mapping is for crews of at most 8");
@@ -467,6 +470,24 @@ __global__ void __launch_bounds__(kT2Threads, CCB_T2_MIN_BLOCKS) cc_step_tpe2_ke
             eflags |= CC_E_WAS_RESET;
             ep_ret = 0.f;
             step = 0;                                               // :97
+          if constexpr (kNp) {
+            // numpy mode: the env's generator (loaded and stored only here), placement of cc_reset_seeded_kernel
+            Pcg64 g = np_load(p.gen[n]);
+#pragma unroll
+            for (int i = 0; i < A; ++i) {
+                int px = 0, py = 0;
+                const bool ok = np_place_agent(g, p, i < B, [&](int cx, int cy) {
+                    const unsigned cell = (unsigned)((cy + 1) * PW + cx + 1);
+                    bool free = true;
+#pragma unroll
+                    for (int j = 0; j < i; ++j) free = free && c[j] != cell;
+                    return free;
+                }, px, py);
+                if (!ok) errbits |= kErrResetStuck;                 // cap hit: keep the last candidate
+                c[i] = (unsigned)((py + 1) * PW + px + 1) & 255u;
+            }
+            p.gen[n] = np_save(g);
+          } else {
 #pragma unroll
             for (int i = 0; i < A; ++i) {
                 unsigned cand = 0;
@@ -486,6 +507,7 @@ __global__ void __launch_bounds__(kT2Threads, CCB_T2_MIN_BLOCKS) cc_step_tpe2_ke
                 if (!ok) errbits |= kErrResetStuck;                 // cap hit: keep the last candidate
                 c[i] = cand & 255u;
             }
+          }
             fl[0] = kM0; fl[1] = kM1;                               // everyone active, nobody done
 #pragma unroll
             for (int k = 0; k < A; ++k) e[k] = lookup(c[k], k);

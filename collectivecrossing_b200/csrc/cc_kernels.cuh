@@ -55,6 +55,11 @@ constexpr unsigned kFull = 0xffffffffu;
 constexpr int kResetAttemptCap = 4096;   // same cap as the oracle
 
 enum Mode { kModeStep = 0, kModeReset = 1, kModePolicy = 2, kModeObserve = 3 };
+// OR-ed into the OBS template argument of a step / reset kernel: placements come from the env's numpy generator
+// (KParams::gen, cc_set_reset_rng) instead of Philox.  A flag of an existing argument, not a new one, so that the
+// Philox instantiations keep their symbols and their code.
+constexpr int kNpReset = 0x100;
+struct Pcg64State;
 enum StatSlot { kStEnvSteps = 0, kStEpisodes, kStTermAll, kStTruncAll, kStArrivals, kStEpLen, kStEpRet, kStRewardSum, kStCount };
 enum ErrBit { kErrInvalidAction = 1, kErrResetStuck = 2 };
 
@@ -119,6 +124,9 @@ struct KParams {
     long long slice_agents;       // elements of one time slice of a per-agent array: n_envs * A
     long long slice_envs;         // ... of a per-env array: n_envs
     long long slice_obs_bytes;    // ... of the observation tensor, in bytes
+    // numpy-mode placements (cc_set_reset_rng): the per-env generators of envs [first, first + n_envs) of the handle;
+    // read by the instantiations that carry kNpReset only.  (Last member: the offsets of the others stay as they were.)
+    Pcg64State *gen;
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -165,6 +173,110 @@ __device__ __forceinline__ bool valid_position(const KParams &p, int x, int y) {
 __device__ __forceinline__ bool in_tram_area(const KParams &p, int x, int y) { return y >= p.D && p.TL <= x && x <= p.TR; }
 // collectivecrossing.py:556-563 is_at_tram_door
 __device__ __forceinline__ bool at_tram_door(const KParams &p, int x, int y) { return y == p.D && (x == p.DL - 1 || x == p.DR + 1); }
+// ---------------------------------------------------------------------------------------------
+// reset(seed=s), bit-exact with the reference's generator: numpy Generator(PCG64(SeedSequence(s)))
+// (gymnasium seeding; collectivecrossing.py:95,105-106,134-137).  One thread per env — the draw
+// stream is inherently sequential.  Restated from numpy's bit_generator.pyx (SeedSequence),
+// _pcg64 / pcg64.h (seeding, XSL-RR 128/64 output, 32-bit buffering) and distributions.c
+// (Lemire bounded uint32), see oracle/cc_oracle.c for the CPU twin.
+// ---------------------------------------------------------------------------------------------
+struct Pcg64 {
+    unsigned long long hi, lo, inc_hi, inc_lo;
+    unsigned buffered;
+    bool has_buffered;
+    __device__ __forceinline__ void advance() {
+        const unsigned long long MH = 2549297995355413924ULL, ML = 4865540595714422341ULL;
+        unsigned long long nlo = lo * ML;
+        unsigned long long nhi = __umul64hi(lo, ML) + hi * ML + lo * MH;
+        unsigned long long slo = nlo + inc_lo;
+        nhi += inc_hi + (slo < nlo ? 1ULL : 0ULL);
+        hi = nhi; lo = slo;
+    }
+    __device__ __forceinline__ unsigned long long next64() {
+        advance();
+        unsigned long long v = hi ^ lo;
+        unsigned rot = (unsigned)(hi >> 58);
+        return (v >> rot) | (v << ((64u - rot) & 63u));
+    }
+    __device__ __forceinline__ unsigned next32() {
+        if (has_buffered) { has_buffered = false; return buffered; }
+        unsigned long long n = next64();
+        has_buffered = true; buffered = (unsigned)(n >> 32);
+        return (unsigned)n;
+    }
+    __device__ __forceinline__ long long integers(long long low, long long high) {  // [low, high)
+        unsigned rng = (unsigned)(high - low) - 1u;
+        if (rng == 0u) return low;
+        unsigned excl = rng + 1u;
+        unsigned long long m = (unsigned long long)next32() * excl;
+        unsigned left = (unsigned)m;
+        if (left < excl) {
+            unsigned thr = (0xFFFFFFFFu - rng) % excl;
+            while (left < thr) { m = (unsigned long long)next32() * excl; left = (unsigned)m; }
+        }
+        return low + (long long)(m >> 32);
+    }
+    __device__ void seed(unsigned long long s) {
+        unsigned ent[2] = {(unsigned)s, (unsigned)(s >> 32)};
+        int n_ent = (s >> 32) ? 2 : 1;
+        unsigned pool[4], hc = 0x43b0d7e5u;
+        auto hashmix = [&](unsigned v) { v ^= hc; hc *= 0x931e8875u; v *= hc; v ^= v >> 16; return v; };
+        auto mix = [](unsigned a, unsigned b) { unsigned r = 0xca01f9ddu * a - 0x4973f715u * b; r ^= r >> 16; return r; };
+        for (int i = 0; i < 4; ++i) pool[i] = hashmix(i < n_ent ? ent[i] : 0u);
+        for (int a = 0; a < 4; ++a)
+            for (int b = 0; b < 4; ++b)
+                if (a != b) pool[b] = mix(pool[b], hashmix(pool[a]));
+        unsigned st[8], hb = 0x8b51f9ddu;
+        for (int i = 0; i < 8; ++i) { unsigned v = pool[i & 3]; v ^= hb; hb *= 0x58f38dedu; v *= hb; v ^= v >> 16; st[i] = v; }
+        unsigned long long w0 = st[0] | ((unsigned long long)st[1] << 32), w1 = st[2] | ((unsigned long long)st[3] << 32);
+        unsigned long long w2 = st[4] | ((unsigned long long)st[5] << 32), w3 = st[6] | ((unsigned long long)st[7] << 32);
+        // pcg_setseq_128_srandom_r(initstate = w0:w1, initseq = w2:w3)
+        inc_hi = (w2 << 1) | (w3 >> 63); inc_lo = (w3 << 1) | 1ULL;
+        hi = 0; lo = 0;
+        advance();
+        unsigned long long slo = lo + w1;
+        hi += w0 + (slo < lo ? 1ULL : 0ULL); lo = slo;
+        advance();
+        has_buffered = false; buffered = 0;
+    }
+};
+
+// persistent generator of one env (what gymnasium keeps in env.np_random): 6 x 8 bytes
+struct Pcg64State { unsigned long long hi, lo, inc_hi, inc_lo, buffered, has_buffered; };
+
+
+__device__ __forceinline__ Pcg64 np_load(const Pcg64State &st) {
+    Pcg64 g;
+    g.hi = st.hi; g.lo = st.lo; g.inc_hi = st.inc_hi; g.inc_lo = st.inc_lo;
+    g.buffered = (unsigned)st.buffered; g.has_buffered = st.has_buffered != 0;
+    return g;
+}
+__device__ __forceinline__ Pcg64State np_save(const Pcg64 &g) {
+    return Pcg64State{g.hi, g.lo, g.inc_hi, g.inc_lo, (unsigned long long)g.buffered, g.has_buffered ? 1ull : 0ull};
+}
+
+// One candidate of reset()'s rejection loop from the env's numpy generator: integers(0, W), integers(0, D) for a
+// boarding agent (collectivecrossing.py:103-117), integers(TL, TR + 1), integers(D, H) for an exiting one (:132-140).
+// Returns the geometric test; the occupancy test against the agents already placed is the caller's.
+__device__ __forceinline__ bool np_candidate(Pcg64 &g, const KParams &p, bool boarding, int &px, int &py) {
+    if (boarding) {
+        px = (int)g.integers(0, p.W); py = (int)g.integers(0, p.D);
+        return valid_position(p, px, py) && !(p.DL <= px && px <= p.DR && py == p.D - 1);
+    }
+    px = (int)g.integers(p.TL, p.TR + 1); py = (int)g.integers(p.D, p.H);
+    return valid_position(p, px, py);
+}
+// reset()'s placement of one agent with the numpy generator: candidates until one passes the geometric test and
+// free(x, y) (no agent j < i stands there).  At kResetAttemptCap attempts the last candidate is kept and false returned.
+// cc_reset_seeded_kernel and the thread-per-env step kernels place every agent through this; the lane-group kernel
+// draws through np_candidate with the same attempt count (its occupancy test is a ballot); tests/native/cc_oracle_np.c restates it.
+template <typename Free>
+__device__ __forceinline__ bool np_place_agent(Pcg64 &g, const KParams &p, bool boarding, Free free, int &px, int &py) {
+    bool ok = false;
+    for (int attempt = 0; attempt < kResetAttemptCap && !ok; ++attempt) ok = np_candidate(g, p, boarding, px, py) && free(px, py);
+    return ok;
+}
+
 // actions.py:18-24 ACTION_TO_DIRECTION
 __device__ __forceinline__ int act_dx(int a) { return (a == CC_ACT_RIGHT) - (a == CC_ACT_LEFT); }
 __device__ __forceinline__ int act_dy(int a) { return (a == CC_ACT_UP) - (a == CC_ACT_DOWN); }
@@ -325,9 +437,12 @@ __device__ __forceinline__ int greedy_decision(int row, unsigned vmask) {
 // ---------------------------------------------------------------------------------------------
 // the fused kernel
 // ---------------------------------------------------------------------------------------------
-template <int LPE, int APL, int OBS, int MODE>
+// OBSF: the obs dtype, with kNpReset for numpy-mode placements (step and reset modes)
+template <int LPE, int APL, int OBSF, int MODE>
 // (two agents per lane: the float32-row instantiation keeps its registers — 122, measured 8 % faster than capped at 128 / 2 CTAs)
-__global__ void __launch_bounds__(kThreads, (MODE != kModeStep) ? 1 : (APL == 1 ? CCB_MIN_BLOCKS : (APL == 2 ? (OBS == CC_OBS_FP32 ? 1 : CCB_MIN_BLOCKS_APL2) : 1))) cc_kernel(const __grid_constant__ KParams p) {
+__global__ void __launch_bounds__(kThreads, (MODE != kModeStep) ? 1 : (APL == 1 ? CCB_MIN_BLOCKS : (APL == 2 ? ((OBSF & ~kNpReset) == CC_OBS_FP32 ? 1 : CCB_MIN_BLOCKS_APL2) : 1))) cc_kernel(const __grid_constant__ KParams p) {
+    constexpr int OBS = OBSF & ~kNpReset;
+    constexpr bool kNp = (OBSF & kNpReset) != 0;
     using TL_ = Tile<LPE, APL>;
     using OT = typename std::conditional<OBS == CC_OBS_FP32, float, int8_t>::type;
     using P2 = typename PairOf<OT>::type;
@@ -886,6 +1001,44 @@ __global__ void __launch_bounds__(kThreads, (MODE != kModeStep) ? 1 : (APL == 1 
         // candidate that passes the geometric test and is not occupied by an agent j < i.  The
         // candidates are drawn by all lanes at once, the acceptance sweep is sequential.
         if ((MODE == kModeStep || MODE == kModeReset) && __any_sync(kFull, need_reset)) {
+          if constexpr (kNp) {
+            // numpy mode: the env's generator is sequential, so the tile's lane 0 holds it, draws the candidates of agent `fin`
+            // one at a time (np_candidate) and broadcasts them; the occupancy ballot accepts a candidate or asks for the next
+            // draw.  Draws, attempt cap and result are those of np_place_agent / cc_reset_seeded_kernel.
+            bool placed[APL];
+#pragma unroll
+            for (int k = 0; k < APL; ++k) placed[k] = false;
+            int fin = need_reset ? 0 : A;  // agents placed so far (tile-uniform)
+            int attempt = 0;               // draws for agent fin (lane 0)
+            Pcg64 g;
+            if (need_reset && T.li == 0) g = np_load(p.gen[n0 + T.tile]);
+            while (__any_sync(kFull, fin < A)) {
+                const bool act_tile = fin < A;
+                unsigned rq = 0;   // bit 31: passes the geometric test, bit 16: attempt cap reached, low 16 bits: packed candidate
+                if (act_tile && T.li == 0) {
+                    int cx, cy;
+                    const bool ok = np_candidate(g, p, fin < p.B, cx, cy);
+                    attempt += 1;
+                    rq = pack_pos(cx, cy) | (ok ? 0x80000000u : 0u) | (attempt >= kResetAttemptCap ? 0x10000u : 0u);
+                }
+                rq = T.tshfl(rq, 0);
+                bool hit = false;
+#pragma unroll
+                for (int s = 0; s < APL; ++s) hit |= placed[s] && pos[s] == (rq & 0xffffu);
+                const unsigned occ = __ballot_sync(kFull, hit) & tile_bits;
+                const bool good = (rq >> 31) && !occ;
+                if (act_tile && (good || (rq & 0x10000u))) {   // accepted, or the cap is hit: the last candidate stays
+                    if (T.li == (fin & (LPE - 1))) {
+#pragma unroll
+                        for (int s = 0; s < APL; ++s) if (s == (fin >> TL_::LOG)) { placed[s] = true; pos[s] = rq & 0xffffu; }
+                    }
+                    if (!good && T.li == 0) errbits |= kErrResetStuck;
+                    fin += 1;
+                    attempt = 0;
+                }
+            }
+            if (need_reset && T.li == 0) p.gen[n0 + T.tile] = np_save(g);
+          } else {
             bool placed[APL], has_cand[APL];
             unsigned cand[APL];
             int attempt[APL];
@@ -948,6 +1101,7 @@ __global__ void __launch_bounds__(kThreads, (MODE != kModeStep) ? 1 : (APL == 1 
                     } else progress = false;
                 }
             }
+          }
             if (need_reset) {
                 step = 0;                                               // :97
 #pragma unroll
@@ -1135,77 +1289,6 @@ __global__ void __launch_bounds__(kThreads, (MODE != kModeStep) ? 1 : (APL == 1 
     if (errbits) atomicOr(p.err, errbits);
 }
 
-// ---------------------------------------------------------------------------------------------
-// reset(seed=s), bit-exact with the reference's generator: numpy Generator(PCG64(SeedSequence(s)))
-// (gymnasium seeding; collectivecrossing.py:95,105-106,134-137).  One thread per env — the draw
-// stream is inherently sequential.  Restated from numpy's bit_generator.pyx (SeedSequence),
-// _pcg64 / pcg64.h (seeding, XSL-RR 128/64 output, 32-bit buffering) and distributions.c
-// (Lemire bounded uint32), see oracle/cc_oracle.c for the CPU twin.
-// ---------------------------------------------------------------------------------------------
-struct Pcg64 {
-    unsigned long long hi, lo, inc_hi, inc_lo;
-    unsigned buffered;
-    bool has_buffered;
-    __device__ __forceinline__ void advance() {
-        const unsigned long long MH = 2549297995355413924ULL, ML = 4865540595714422341ULL;
-        unsigned long long nlo = lo * ML;
-        unsigned long long nhi = __umul64hi(lo, ML) + hi * ML + lo * MH;
-        unsigned long long slo = nlo + inc_lo;
-        nhi += inc_hi + (slo < nlo ? 1ULL : 0ULL);
-        hi = nhi; lo = slo;
-    }
-    __device__ __forceinline__ unsigned long long next64() {
-        advance();
-        unsigned long long v = hi ^ lo;
-        unsigned rot = (unsigned)(hi >> 58);
-        return (v >> rot) | (v << ((64u - rot) & 63u));
-    }
-    __device__ __forceinline__ unsigned next32() {
-        if (has_buffered) { has_buffered = false; return buffered; }
-        unsigned long long n = next64();
-        has_buffered = true; buffered = (unsigned)(n >> 32);
-        return (unsigned)n;
-    }
-    __device__ __forceinline__ long long integers(long long low, long long high) {  // [low, high)
-        unsigned rng = (unsigned)(high - low) - 1u;
-        if (rng == 0u) return low;
-        unsigned excl = rng + 1u;
-        unsigned long long m = (unsigned long long)next32() * excl;
-        unsigned left = (unsigned)m;
-        if (left < excl) {
-            unsigned thr = (0xFFFFFFFFu - rng) % excl;
-            while (left < thr) { m = (unsigned long long)next32() * excl; left = (unsigned)m; }
-        }
-        return low + (long long)(m >> 32);
-    }
-    __device__ void seed(unsigned long long s) {
-        unsigned ent[2] = {(unsigned)s, (unsigned)(s >> 32)};
-        int n_ent = (s >> 32) ? 2 : 1;
-        unsigned pool[4], hc = 0x43b0d7e5u;
-        auto hashmix = [&](unsigned v) { v ^= hc; hc *= 0x931e8875u; v *= hc; v ^= v >> 16; return v; };
-        auto mix = [](unsigned a, unsigned b) { unsigned r = 0xca01f9ddu * a - 0x4973f715u * b; r ^= r >> 16; return r; };
-        for (int i = 0; i < 4; ++i) pool[i] = hashmix(i < n_ent ? ent[i] : 0u);
-        for (int a = 0; a < 4; ++a)
-            for (int b = 0; b < 4; ++b)
-                if (a != b) pool[b] = mix(pool[b], hashmix(pool[a]));
-        unsigned st[8], hb = 0x8b51f9ddu;
-        for (int i = 0; i < 8; ++i) { unsigned v = pool[i & 3]; v ^= hb; hb *= 0x58f38dedu; v *= hb; v ^= v >> 16; st[i] = v; }
-        unsigned long long w0 = st[0] | ((unsigned long long)st[1] << 32), w1 = st[2] | ((unsigned long long)st[3] << 32);
-        unsigned long long w2 = st[4] | ((unsigned long long)st[5] << 32), w3 = st[6] | ((unsigned long long)st[7] << 32);
-        // pcg_setseq_128_srandom_r(initstate = w0:w1, initseq = w2:w3)
-        inc_hi = (w2 << 1) | (w3 >> 63); inc_lo = (w3 << 1) | 1ULL;
-        hi = 0; lo = 0;
-        advance();
-        unsigned long long slo = lo + w1;
-        hi += w0 + (slo < lo ? 1ULL : 0ULL); lo = slo;
-        advance();
-        has_buffered = false; buffered = 0;
-    }
-};
-
-// persistent generator of one env (what gymnasium keeps in env.np_random): 6 x 8 bytes
-struct Pcg64State { unsigned long long hi, lo, inc_hi, inc_lo, buffered, has_buffered; };
-
 // seeds != nullptr: reset(seed=seeds[n]) — a fresh generator per env (gymnasium Env.reset(seed=s));
 // seeds == nullptr: reset() — every env keeps drawing from its stored generator.
 // (a plain function, not a template: defined in the one translation unit that sets CCB_WITH_RESET_SEEDED)
@@ -1215,33 +1298,23 @@ __global__ void __launch_bounds__(128) cc_reset_seeded_kernel(const __grid_const
     if (n >= p.n_envs) return;
     Pcg64 g;
     if (seeds) g.seed((unsigned long long)seeds[n]);
-    else {
-        const Pcg64State st = gen[n];
-        g.hi = st.hi; g.lo = st.lo; g.inc_hi = st.inc_hi; g.inc_lo = st.inc_lo;
-        g.buffered = (unsigned)st.buffered; g.has_buffered = st.has_buffered != 0;
-    }
+    else g = np_load(gen[n]);
     int8_t *x = p.x + n * p.A, *y = p.y + n * p.A;
     int stuck = 0;
     for (int i = 0; i < p.A; ++i) {
         int px = 0, py = 0;
-        bool ok = false;
-        for (int attempt = 0; attempt < kResetAttemptCap && !ok; ++attempt) {
-            if (i < p.B) {
-                px = (int)g.integers(0, p.W); py = (int)g.integers(0, p.D);
-                ok = valid_position(p, px, py) && !(p.DL <= px && px <= p.DR && py == p.D - 1);
-            } else {
-                px = (int)g.integers(p.TL, p.TR + 1); py = (int)g.integers(p.D, p.H);
-                ok = valid_position(p, px, py);
-            }
-            for (int j = 0; ok && j < i; ++j) ok = !(x[j] == px && y[j] == py);
-        }
+        const bool ok = np_place_agent(g, p, i < p.B, [&](int cx, int cy) {
+            for (int j = 0; j < i; ++j)
+                if (x[j] == cx && y[j] == cy) return false;
+            return true;
+        }, px, py);
         if (!ok) stuck = 1;
         x[i] = (int8_t)px; y[i] = (int8_t)py;
         p.flags[n * p.A + i] = CC_F_ACTIVE;
     }
     p.step[n] = 0;
     p.ep_ret[n] = 0.f;
-    gen[n] = Pcg64State{g.hi, g.lo, g.inc_hi, g.inc_lo, (unsigned long long)g.buffered, g.has_buffered ? 1ull : 0ull};
+    gen[n] = np_save(g);
     if (stuck) atomicOr(p.err, kErrResetStuck);
 }
 #endif  // CCB_WITH_RESET_SEEDED

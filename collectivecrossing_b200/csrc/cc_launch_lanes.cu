@@ -25,26 +25,33 @@ int launch_t(cc_handle *h, const KParams &p, cudaStream_t s) {
     if (grid < 1) grid = 1;
     kern<<<grid, ccb::kThreads, smem, s>>>(p);
     CC_CUDA(cudaGetLastError());
-    if (MODE == ccb::kModeStep) snprintf(h->last_kernel, sizeof h->last_kernel, "ccb::cc_kernel<%d,%d,%d,step>", LPE, APL, OBS);
+    if (MODE == ccb::kModeStep) snprintf(h->last_kernel, sizeof h->last_kernel, "ccb::cc_kernel<%d,%d,%d,step>", LPE, APL, OBS);   // (OBS | 256: numpy placements)
     h->launches += 1;
     return CC_OK;
 }
 
-template <int LPE, int APL, int MODE>
-int launch_obs(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s) {
+// F: 0, or ccb::kNpReset for the numpy-mode step / reset instantiations (KParams::gen set)
+template <int LPE, int APL, int MODE, int F>
+int launch_obs_f(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s) {
     if constexpr (MODE == ccb::kModePolicy) {
         return launch_t<LPE, APL, CC_OBS_NONE, MODE>(h, p, s);
     } else {
         switch (obs_dtype) {
         case CC_OBS_NONE:
             if constexpr (MODE == ccb::kModeObserve) return cc_fail(CC_ERR_INVALID_ARG, "observe needs an observation dtype");
-            else return launch_t<LPE, APL, CC_OBS_NONE, MODE>(h, p, s);
-        case CC_OBS_INT8: return launch_t<LPE, APL, CC_OBS_INT8, MODE>(h, p, s);
-        case CC_OBS_FP32: return launch_t<LPE, APL, CC_OBS_FP32, MODE>(h, p, s);
-        case CC_OBS_TABLE: return launch_t<LPE, APL, CC_OBS_TABLE, MODE>(h, p, s);
+            else return launch_t<LPE, APL, CC_OBS_NONE | F, MODE>(h, p, s);
+        case CC_OBS_INT8: return launch_t<LPE, APL, CC_OBS_INT8 | F, MODE>(h, p, s);
+        case CC_OBS_FP32: return launch_t<LPE, APL, CC_OBS_FP32 | F, MODE>(h, p, s);
+        case CC_OBS_TABLE: return launch_t<LPE, APL, CC_OBS_TABLE | F, MODE>(h, p, s);
         }
         return cc_fail(CC_ERR_INVALID_ARG, "unknown obs_dtype %d", obs_dtype);
     }
+}
+template <int LPE, int APL, int MODE>
+int launch_obs(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s) {
+    if constexpr (MODE == ccb::kModeStep || MODE == ccb::kModeReset)
+        if (p.gen) return launch_obs_f<LPE, APL, MODE, ccb::kNpReset>(h, p, obs_dtype, s);
+    return launch_obs_f<LPE, APL, MODE, 0>(h, p, obs_dtype, s);
 }
 
 template <int MODE>

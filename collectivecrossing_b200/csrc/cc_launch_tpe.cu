@@ -19,7 +19,7 @@ using ccb::KParams;
 
 template <int A, int OBS>
 int launch_tpe_t(cc_handle *h, KParams p, cudaStream_t s) {
-    using L = ccb::TpeLayout<A, OBS>;
+    using L = ccb::TpeLayout<A, OBS & ~ccb::kNpReset>;
     auto kern = ccb::cc_step_tpe_kernel<A, OBS>;
     p.n_groups = (p.n_envs + 31) / 32;
     // greedy / waiting: a private lattice bitmap per thread while the lattice is small (README: 6 words)
@@ -55,7 +55,7 @@ int launch_tpe_t(cc_handle *h, KParams p, cudaStream_t s) {
 // cc_step_tpe2_kernel: small lattices, compact output modes (cc_kernel_tpe2.cuh)
 template <int A, int OBS, int BT = -1>
 int launch_tpe2_t(cc_handle *h, KParams p, cudaStream_t s) {
-    using L = ccb::T2Layout<A, OBS>;
+    using L = ccb::T2Layout<A, OBS & ~ccb::kNpReset>;
     auto kern = ccb::cc_step_tpe2_kernel<A, OBS, BT>;
     int rc0 = cc_t2_ensure_tables(h, p, s);
     if (rc0 != CC_OK) return rc0;
@@ -100,27 +100,32 @@ bool tpe2_eligible(const KParams &p, int obs_dtype) {
 
 }  // namespace
 
-#define CCB_TPE2_CASES(A_)                                                                  \
-    case A_ * 32 + CC_OBS_NONE: return launch_tpe2_t<A_, CC_OBS_NONE>(h, p, s);                 \
-    case A_ * 32 + CC_OBS_TABLE: return launch_tpe2_t<A_, CC_OBS_TABLE>(h, p, s);
-#define CCB_TPE2_CASES_EVEN(A_)                                                             \
-    CCB_TPE2_CASES(A_)                                                                      \
-    case A_ * 32 + CC_OBS_FP32: return launch_tpe2_t<A_, CC_OBS_FP32>(h, p, s);
-#define CCB_TPE_CASES(A_)                                                                   \
-    case A_ * 32 + CC_OBS_NONE: return launch_tpe_t<A_, CC_OBS_NONE>(h, p, s);                  \
-    case A_ * 32 + CC_OBS_TABLE: return launch_tpe_t<A_, CC_OBS_TABLE>(h, p, s);                \
-    case A_ * 32 + CC_OBS_FP32: return launch_tpe_t<A_, CC_OBS_FP32>(h, p, s);
+// F: 0, or ccb::kNpReset for the numpy-mode instantiations (KParams::gen set)
+#define CCB_TPE2_CASES(A_, F)                                                               \
+    case A_ * 32 + CC_OBS_NONE: return launch_tpe2_t<A_, CC_OBS_NONE | F>(h, p, s);             \
+    case A_ * 32 + CC_OBS_TABLE: return launch_tpe2_t<A_, CC_OBS_TABLE | F>(h, p, s);
+#define CCB_TPE2_CASES_EVEN(A_, F)                                                          \
+    CCB_TPE2_CASES(A_, F)                                                                   \
+    case A_ * 32 + CC_OBS_FP32: return launch_tpe2_t<A_, CC_OBS_FP32 | F>(h, p, s);
+#define CCB_TPE_CASES(A_, F)                                                                \
+    case A_ * 32 + CC_OBS_NONE: return launch_tpe_t<A_, CC_OBS_NONE | F>(h, p, s);              \
+    case A_ * 32 + CC_OBS_TABLE: return launch_tpe_t<A_, CC_OBS_TABLE | F>(h, p, s);            \
+    case A_ * 32 + CC_OBS_FP32: return launch_tpe_t<A_, CC_OBS_FP32 | F>(h, p, s);
 
 #if CCB_TPE_PART == 0
-int cc_launch_tpe_part0(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s) {
+template <int F>
+int launch_tpe_part0(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s) {
     if (tpe2_eligible(p, obs_dtype)) {
-        switch (p.A * 32 + obs_dtype) { CCB_TPE2_CASES(1) CCB_TPE2_CASES_EVEN(2) CCB_TPE2_CASES(3) CCB_TPE2_CASES_EVEN(4) }
+        switch (p.A * 32 + obs_dtype) { CCB_TPE2_CASES(1, F) CCB_TPE2_CASES_EVEN(2, F) CCB_TPE2_CASES(3, F) CCB_TPE2_CASES_EVEN(4, F) }
     }
     switch (p.A * 32 + obs_dtype) {
-        CCB_TPE_CASES(1) CCB_TPE_CASES(2) CCB_TPE_CASES(3) CCB_TPE_CASES(4)
-    case 8 * 32 + CC_OBS_INT8: return launch_tpe_t<8, CC_OBS_INT8>(h, p, s);
+        CCB_TPE_CASES(1, F) CCB_TPE_CASES(2, F) CCB_TPE_CASES(3, F) CCB_TPE_CASES(4, F)
+    case 8 * 32 + CC_OBS_INT8: return launch_tpe_t<8, CC_OBS_INT8 | F>(h, p, s);
     }
     return cc_fail(CC_ERR_UNSUPPORTED, "no thread-per-env kernel for %d agents, obs_dtype %d", p.A, obs_dtype);
+}
+int cc_launch_tpe_part0(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s) {
+    return p.gen ? launch_tpe_part0<ccb::kNpReset>(h, p, obs_dtype, s) : launch_tpe_part0<0>(h, p, obs_dtype, s);
 }
 #else
 int cc_launch_tpe_part0(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s);
@@ -136,9 +141,10 @@ int cc_t2_ensure_tables(cc_handle *h, const KParams &p, cudaStream_t s) {
     return CC_OK;
 }
 
-int cc_launch_tpe(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s) {
+template <int F>
+int launch_tpe_part1(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s) {
     if (tpe2_eligible(p, obs_dtype)) {
-        if (p.A == 8 && p.B == 5) {   // the README crew: boarding / exiting split known at compile time
+        if (F == 0 && p.A == 8 && p.B == 5) {   // the README crew: boarding / exiting split known at compile time (Philox placements)
             switch (obs_dtype) {
             case CC_OBS_NONE: return launch_tpe2_t<8, CC_OBS_NONE, 5>(h, p, s);
             case CC_OBS_TABLE: return launch_tpe2_t<8, CC_OBS_TABLE, 5>(h, p, s);
@@ -147,13 +153,16 @@ int cc_launch_tpe(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s)
             }
         }
         switch (p.A * 32 + obs_dtype) {
-            CCB_TPE2_CASES(5) CCB_TPE2_CASES_EVEN(6) CCB_TPE2_CASES(7) CCB_TPE2_CASES_EVEN(8)
-        case 8 * 32 + CC_OBS_INT8: return launch_tpe2_t<8, CC_OBS_INT8>(h, p, s);
+            CCB_TPE2_CASES(5, F) CCB_TPE2_CASES_EVEN(6, F) CCB_TPE2_CASES(7, F) CCB_TPE2_CASES_EVEN(8, F)
+        case 8 * 32 + CC_OBS_INT8: return launch_tpe2_t<8, CC_OBS_INT8 | F>(h, p, s);
         }
     }
     switch (p.A * 32 + obs_dtype) {
-        CCB_TPE_CASES(5) CCB_TPE_CASES(6) CCB_TPE_CASES(7) CCB_TPE_CASES(8)
+        CCB_TPE_CASES(5, F) CCB_TPE_CASES(6, F) CCB_TPE_CASES(7, F) CCB_TPE_CASES(8, F)
     }
     return cc_launch_tpe_part0(h, p, obs_dtype, s);
+}
+int cc_launch_tpe(cc_handle *h, const KParams &p, int obs_dtype, cudaStream_t s) {
+    return p.gen ? launch_tpe_part1<ccb::kNpReset>(h, p, obs_dtype, s) : launch_tpe_part1<0>(h, p, obs_dtype, s);
 }
 #endif

@@ -76,7 +76,8 @@ class ShardedCollectiveCrossing:
     """``total_envs`` envs split over the ranks of the default process group.
 
     ``env_factory(config, num_envs, global_env_offset=..., seed=..., **kw)`` builds the rank-local
-    env; by default the CUDA ``BatchedCollectiveCrossing`` on ``cuda:LOCAL_RANK``.
+    env; by default the CUDA ``BatchedCollectiveCrossing`` on ``cuda:LOCAL_RANK``.  ``env_kwargs`` (``obs_dtype``,
+    ``reset_rng``, ...) go to every rank's env.
     """
 
     def __init__(self, config: Any, total_envs: int, *, seed: int = 0, device: Any = None,

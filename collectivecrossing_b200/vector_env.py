@@ -59,14 +59,15 @@ class VectorCollectiveCrossing:
     """N CollectiveCrossing envs for a learner; see the module docstring."""
 
     def __init__(self, config: Any, num_envs: int, device: Any = "cuda:0", *, seed: int = 0, auto_reset: bool = True,
-                 global_env_offset: int = 0):
+                 global_env_offset: int = 0, reset_rng: str = "philox"):
         if isinstance(config, dict):  # RLlib env_config dicts
             from .configs import CollectiveCrossingConfig
 
             config = CollectiveCrossingConfig(**config)
         self.config = config
         self.env = BatchedCollectiveCrossing(config, num_envs, device, seed=seed, obs_dtype="float32", reward_dtype="float32",
-                                             auto_reset=auto_reset, with_info=True, global_env_offset=global_env_offset)
+                                             auto_reset=auto_reset, with_info=True, global_env_offset=global_env_offset,
+                                             reset_rng=reset_rng)
         self.num_envs = self.env.num_envs
         self.num_agents = self.env.num_agents
         self.num_boarding = config.num_boarding_agents
@@ -92,8 +93,10 @@ class VectorCollectiveCrossing:
 
     # ---- reset / step ----------------------------------------------------------------------------------
     def reset(self, *, seed: int | torch.Tensor | None = None) -> torch.Tensor:
-        """All envs.  ``seed=None``: counter-based placement; an int ``s``: env n is reset like the
-        reference's ``reset(seed=s+n)`` (numpy-exact PCG64 placement); a tensor: one seed per env."""
+        """All envs.  ``seed=None``: counter-based placement (``reset_rng="numpy"``: every env continues its numpy
+        generator, the reference's ``reset()``); an int ``s``: env n is reset like the reference's ``reset(seed=s+n)``
+        (numpy-exact PCG64 placement); a tensor: one seed per env.  With ``reset_rng="numpy"``, ``reset(seed=s)``
+        followed by ``step`` with auto-reset reproduces N reference envs seeded ``s + n``, episode after episode."""
         if seed is None:
             return self.env.reset()
         if not torch.is_tensor(seed):

@@ -261,7 +261,8 @@ int cc_rollout(cc_handle *h, const cc_step_io *io, int32_t n_steps, void *stream
 int cc_rollout_fused(cc_handle *h, const cc_step_io *io, int32_t n_steps, void *stream);
 
 /* Replaces CollectiveCrossingEnv.reset (collectivecrossing.py:91-159): rejection-sampled
- * placement with the handle's counter-based RNG.  mask: [N] uint8 nullable (NULL = all envs).
+ * placement with the handle's counter-based RNG, or with each env's numpy generator under
+ * CC_RESET_RNG_NUMPY (cc_set_reset_rng).  mask: [N] uint8 nullable (NULL = all envs).
  * obs nullable; written for the reset envs only when given. */
 int cc_reset(cc_handle *h, const uint8_t *mask, void *obs, int32_t obs_dtype, void *stream);
 
@@ -281,6 +282,21 @@ int cc_get_rng_state(cc_handle *h, uint64_t *out, void *stream);
 int cc_set_rng_state(cc_handle *h, const uint64_t *in, void *stream);
 /* 1 once the generators hold a stream (after cc_reset_seeded(seeds) or cc_set_rng_state) */
 int32_t cc_rng_seeded(const cc_handle *h);
+
+/* Where UNSEEDED placements come from: the auto-reset of cc_step, cc_rollout, cc_rollout_fused, cc_step_host and
+ * cc_rollout_host, and cc_reset(mask).
+ *   CC_RESET_RNG_PHILOX (default): the counter-based generator keyed (seed, global env, t) — new functionality, the
+ *       reference has no auto-reset.
+ *   CC_RESET_RNG_NUMPY: the reference's reset() without a seed — env n draws from its own numpy generator (the one
+ *       cc_reset_seeded keeps, checkpointed by cc_get_rng_state) and advances it, exactly as cc_reset_seeded(NULL)
+ *       does for that env.  N envs each reset(seed=s_n) once and then stepped with reset() on "__all__" reproduce the
+ *       reference episode after episode.  A call that may place envs (auto_reset != 0, or cc_reset) fails with
+ *       CC_ERR_INVALID_ARG before it enqueues anything until the generators are seeded (cc_reset_seeded(seeds) or
+ *       cc_set_rng_state).  The step counter t advances as in Philox mode, so random-policy actions are the same.
+ * Results of one mode never depend on the kernel mapping (cc_set_kernel_variant) or on the host path's chunking. */
+enum { CC_RESET_RNG_PHILOX = 0, CC_RESET_RNG_NUMPY = 1 };
+int cc_set_reset_rng(cc_handle *h, int32_t source);
+int32_t cc_reset_rng(const cc_handle *h);
 
 /* The baseline policies alone (greedy_policy.py:33-88, waiting_policy.py:33-72) on the
  * current state: actions_out [N,A] int8; agents that are done or inactive get CC_ACT_WAIT. */
