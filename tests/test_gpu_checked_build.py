@@ -21,7 +21,8 @@ def test_parity_cases_pass_in_the_checked_build():
     env = dict(os.environ, CCB200_LIB=str(CHECKED))
     sel = ["tests/test_gpu_small_lattice.py", "tests/test_gpu_host_path.py::test_table_mode_matches_oracle",
            "tests/test_gpu_parity.py::test_device_matches_oracle_with_auto_reset", "tests/test_gpu_parity.py::test_fused_rollout_equals_repeated_steps",
-           "tests/test_gpu_parity.py::test_thread_per_env_kernel_replays_golden"]
+           "tests/test_gpu_parity.py::test_thread_per_env_kernel_replays_golden",
+           "tests/test_gpu_geometry_edges.py"]
     proc = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu", "-p", "no:cacheprovider", *sel], cwd=ROOT, env=env,
                           capture_output=True, text=True, timeout=1500)
     tail = (proc.stdout + proc.stderr)[-3000:]
